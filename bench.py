@@ -29,6 +29,13 @@ One step = parse the text into the (vendor,device) table and join the 2^20 keys 
   --impl reference   the reference's own algorithm (getDeviceName: one linear rescan of the
              text per key, pkg/device_plugin/device_plugin.go:208-275) restated in C
              (oracle/, Go toolchain absent), all host threads, bounded sample per step.
+  --dump-outputs DIR   after the timed steps, rank 0 writes what the last timed step returned as
+             float64 .npy files (same inputs on every run, so two builds compare file for file):
+             table_key / table_line_off   the table in file order (kxpu_table_export),
+             join_line_off                per key, the line offset of the row it hit (-1 = miss).
+             Row handles are opaque numbers, so the join is written as the line each handle stands for.
+
+The tree may be read-only: bench.py uses the libraries build() made and writes nothing there.
 """
 import argparse
 import json
@@ -38,6 +45,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True  # no __pycache__ in the tree
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -182,7 +190,6 @@ def run_reference(args, rank, out_fd):
     import kxpu_b200  # noqa: F401  (workloads only; no GPU context is created on this arm)
     from kxpu_b200 import workloads as W
     from oracle import oracle as O
-    O.build()
     text = W.load_pci_ids()
     text_x = np.tile(np.frombuffer(text, np.uint8), COPIES)
     present = O.table_build(text)["key"]
@@ -247,7 +254,12 @@ def main():
     ap.add_argument("--no-second-mode", action="store_true", help="N > 1: measure only --scaling, not the other mode beside it")
     ap.add_argument("--settle-ms", type=float, default=400.0,
                     help="untimed extra warm-up (clock settling + nvidia-smi samples); the step count is reported in the line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -348,8 +360,18 @@ def main():
         for k in ("d_text", "d_keys", "d_rows"):
             kx.dev_free(w[k])
 
-    def measure(w, steps, warmup, settle_ms, sampler=None):
-        """Device-timed K steps (max over ranks) + per-kernel device times from separate passes."""
+    def step_result(t, d_rows):
+        """The table of a step in file order, the row handles of all NQ keys and the line offset each
+        handle stands for (-1 = miss)."""
+        tk, to, tr = kx.table_export(t)
+        got = kx.download(d_rows, NQ * 4, np.int32)
+        line_of_row = np.full(t.rows + 1, -1, np.int64)
+        line_of_row[tr] = to.astype(np.int64)
+        return tk, to, got, np.where(got >= 0, line_of_row[np.maximum(got, 0)], -1)
+
+    def measure(w, steps, warmup, settle_ms, sampler=None, keep_outputs=False):
+        """Device-timed K steps (max over ranks) + per-kernel device times from separate passes.
+        keep_outputs: also return what the last timed step computed (read after the timer stops)."""
         for _ in range(warmup):
             w["step"]().free()
         kx.sync()
@@ -365,12 +387,18 @@ def main():
         kx.set_stage_timing(False)  # the per-stage events are for the separate per-kernel passes below
         kx.timer_begin()
         t_wall = time.time()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             w["step"]().free()
+        last = w["step"]()
         ms_total = kx.timer_end()
         kx.set_stage_timing(True)
         barrier()
         wall_ms = (time.time() - t_wall) * 1e3
+        outputs = None
+        if keep_outputs:
+            tk, to, _, got_line = step_result(last, w["d_rows"])
+            outputs = {"table_key": tk, "table_line_off": to, "join_line_off": got_line}
+        last.free()
         launches = kx.launch_count() - launches0
         clocks = sampler.stop() if sampler is not None else None
         km = {k: [] for k in ("parse", "parse_resolve", "finalize", "merge", "lookup")}
@@ -385,7 +413,7 @@ def main():
         ms_step = max_over_ranks(ms_total) / steps
         return dict(ms_per_step=ms_step, value=w["job_bytes"] / (ms_step * 1e-3) / 1e9, wall_ms_per_step=wall_ms / steps,
                     launches=int(launches), settle_steps=settle, clocks=clocks,
-                    kernel_ms={k: float(np.mean(v)) for k, v in km.items()})
+                    kernel_ms={k: float(np.mean(v)) for k, v in km.items()}, outputs=outputs)
 
     def measure_e2e(w, steps):
         """The same step from HOST buffers: pinned text (shard) -> H2D, kernels, D2H of the row handles."""
@@ -414,17 +442,12 @@ def main():
         """Every rank: table hash + join result vs the oracle's table of the WHOLE text (rank 0 builds it
         with kxo_table_build on the 1.458 GB buffer, outside every timed region)."""
         t = w["step"]()
-        tk, to, tr = kx.table_export(t)
-        got = kx.download(w["d_rows"], NQ * 4, np.int32)
-        line_of_row = np.full(t.rows + 1, -1, np.int64)
-        line_of_row[tr] = to.astype(np.int64)
-        got_line = np.where(got >= 0, line_of_row[np.maximum(got, 0)], -1)
+        tk, to, got, got_line = step_result(t, w["d_rows"])
         t.free()
         ok, detail = True, {}
         if w["kind"] == "strong":
             if rank == 0:
                 from oracle import oracle as O
-                O.build()
                 t0 = time.time()
                 orows = O.table_build(h_text)
                 detail["oracle_s"] = time.time() - t0
@@ -433,7 +456,6 @@ def main():
                 detail["rows"] = int(len(orows)); detail["hits"] = int((got >= 0).sum())
         else:  # weak: the logical text is x(1000*world); first occurrence wins -> the single-copy table; own keys
             from oracle import oracle as O
-            O.build()
             orows = O.table_build(text)
             ok = bool(np.array_equal(tk, orows["key"]) and np.array_equal(to, orows["line_off"]))
             ok = ok and bool(np.array_equal(got_line, expected_lines(orows, w["h_keys"])))
@@ -457,7 +479,8 @@ def main():
     results = {}
     for i, mode in enumerate(modes):
         w = make_strong() if mode == "strong" else make_weak()
-        r = measure(w, args.steps, args.warmup, args.settle_ms, sampler if (i == 0 and rank == 0) else None)
+        r = measure(w, args.steps, args.warmup, args.settle_ms, sampler if (i == 0 and rank == 0) else None,
+                    keep_outputs=bool(args.dump_outputs) and i == 0 and rank == 0)
         r["e2e"] = measure_e2e(w, args.e2e_steps)
         r["e2e"].pop("rows")
         ok, detail = check_parity(w)
@@ -482,6 +505,10 @@ def main():
         else:
             results["_w"] = w
     head = results[args.scaling]
+    if head["outputs"] is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in head["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a.astype(np.float64))
 
     line = None
     if rank == 0:
@@ -534,7 +561,6 @@ def main():
             line["aux"] = aux_configs(kx, K, W, text, present, peak)
         if rank == 0 and not args.no_cpu_baseline:
             from oracle import oracle as O
-            O.build()
             use_all_cpus()
             threads = host_threads()
             nk = max(threads * 16, 64)  # ~10 s wall on all host cores

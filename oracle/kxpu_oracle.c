@@ -610,7 +610,8 @@ size_t kxo_table_build_mt(const uint8_t *text, size_t n, int threads, kxo_row *r
             const kxo_row *r = &jobs[t].rows[i];
             /* a top-level line is a valid anchor only in front of the cut-off, a row only in front of it too */
             if (r->anchor_off == gfirst[r->key >> 16] && r->line_off < trunc) {
-                if (rows_out && nr < cap) rows_out[nr] = *r;
+                /* field by field, like kxo_table_build: a struct copy would carry the uninitialised padding after key */
+                if (rows_out && nr < cap) { rows_out[nr].key = r->key; rows_out[nr].line_off = r->line_off; rows_out[nr].anchor_off = r->anchor_off; }
                 nr++;
             }
         }

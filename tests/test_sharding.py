@@ -227,7 +227,7 @@ def test_two_gpu_process_per_rank(no_p2p):
     """One process per rank under torchrun: CUDA-IPC peer memory, and the NCCL transport (KXPU_NO_P2P=1)."""
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2); the exchange itself is covered on one GPU above")
+        pytest.skip("needs 2 GPUs; the exchange itself is covered on one GPU above")
     env = dict(os.environ, KXPU_NO_P2P=no_p2p) if no_p2p == "1" else dict(os.environ)
     env.pop("KXPU_NO_P2P", None) if no_p2p == "0" else None
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr", "127.0.0.1",

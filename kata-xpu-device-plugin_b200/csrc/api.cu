@@ -73,8 +73,6 @@ int32_t kx_ctx_create_on(int32_t ordinal, kxpu_ctx **out) {
     const char *fr = getenv("KXPU_RCH");
     c->force_rch = (fr && fr[0] >= '1' && fr[0] <= '8' && !fr[1]) ? fr[0] - '0' : 0;
     c->no_small = getenv("KXPU_NO_SMALL") != nullptr;
-    c->no_zero_copy = getenv("KXPU_NO_ZERO_COPY") != nullptr;
-    if (const char *sw = getenv("KXPU_SCAN_W")) { const int v = atoi(sw); c->force_scan_w = (v == 8 || v == 16 || v == 32) ? v : 0; }
     *out = c;
     return KXPU_OK;
 }
@@ -425,17 +423,24 @@ int32_t kx_launch_trunc(kxpu_ctx *ctx, kxpu_table *t, const uint8_t *d_text, siz
     return KXPU_OK;
 }
 
-int32_t kx_launch_finalize(kxpu_ctx *ctx, kxpu_table *t, const uint8_t *d_text, size_t n, unsigned long long base,
-                           const kxx::MinView *mv, const kxx::WaitSpec *wait, const KxSlabOut *slab) {
+// finalize of table t over text[0, n) at global offset base: validity against the table's own first anchors and
+// cut-off, rows and names into the table's arrays
+static kxparse::FinalizeParams finalize_params(const kxpu_table *t, const uint8_t *text, size_t n, unsigned long long base) {
     kxparse::FinalizeParams F;
     memset(&F, 0, sizeof F);
-    if (wait) F.wait = *wait;
-    F.text = d_text; F.n = n; F.base = base; F.tab = t->dev;
-    if (mv) F.mv = *mv;
-    else { F.mv.a = t->dev.vendor_first; F.mv.stride = 0; F.mv.n = 1; F.mv.trunc1 = t->dev.trunc; }
+    F.text = text; F.n = n; F.base = base; F.tab = t->dev;
+    F.mv.a = t->dev.vendor_first; F.mv.stride = 0; F.mv.n = 1; F.mv.trunc1 = t->dev.trunc;
     F.row_key = t->row_key; F.row_line = t->row_line; F.row_anchor = t->row_anchor;
     F.row_name_off = t->row_name_off; F.row_name_len = t->row_name_len;
     F.blob = t->blob; F.blob_cap = t->blob_cap;
+    return F;
+}
+
+int32_t kx_launch_finalize(kxpu_ctx *ctx, kxpu_table *t, const uint8_t *d_text, size_t n, unsigned long long base,
+                           const kxx::MinView *mv, const kxx::WaitSpec *wait, const KxSlabOut *slab) {
+    kxparse::FinalizeParams F = finalize_params(t, d_text, n, base);
+    if (wait) F.wait = *wait;
+    if (mv) F.mv = *mv;
     if (slab) {
         F.slab_rows = reinterpret_cast<kxx::SlabRow *>(slab->rows); F.slab_rows_cap = slab->rows_cap;
         F.blob = slab->blob; F.blob_cap = slab->blob_cap;
@@ -445,7 +450,6 @@ int32_t kx_launch_finalize(kxpu_ctx *ctx, kxpu_table *t, const uint8_t *d_text, 
     // validity + names: a warp scans scan_w table slots per step, persistent grid.  Small tables: 8 slots per
     // warp keep every warp of the grid busy with one short chain; big ones scan 32 and work off full batches
     F.scan_w = t->cap >= (1u << 19) ? 32u : 8u;
-    if (ctx->force_scan_w) F.scan_w = (uint32_t)ctx->force_scan_w;
     const unsigned batches = (t->cap + 1 + F.scan_w - 1) / F.scan_w;
     const unsigned grid = std::min<unsigned>((batches + kxparse::SF_WARPS - 1) / kxparse::SF_WARPS, 8u * ctx->sm_count);
     kxparse::select_finalize_kernel<<<grid, kxparse::SF_WARPS * 32, 0, ctx->stream>>>(F);
@@ -508,12 +512,8 @@ static int32_t launch_small(kxpu_ctx *ctx, kxpu_table *t, const uint8_t *d_text,
     P.num_chunks = (uint32_t)((n + CW - 1) / CW);
     P.tma_limit = n >= (size_t)STG_BYTES ? (uint32_t)((n - STG_BYTES) / CW) + 1u : 0u;
     P.state = t->range_words;
+    P.F = finalize_params(t, d_text, n, 0);
     FinalizeParams &F = P.F;
-    F.text = d_text; F.n = n; F.base = 0; F.tab = t->dev;
-    F.mv.a = t->dev.vendor_first; F.mv.stride = 0; F.mv.n = 1; F.mv.trunc1 = t->dev.trunc;
-    F.row_key = t->row_key; F.row_line = t->row_line; F.row_anchor = t->row_anchor;
-    F.row_name_off = t->row_name_off; F.row_name_len = t->row_name_len;
-    F.blob = t->blob; F.blob_cap = t->blob_cap;
     if (join) { P.keys = join->d_keys; P.nq = join->n; P.rows_out = join->d_rows; }
     if (join && join->src_text) { P.text_src = join->src_text; P.h_ctl = ctx->h_ctl; }
     void *args[] = {&P};
@@ -522,18 +522,17 @@ static int32_t launch_small(kxpu_ctx *ctx, kxpu_table *t, const uint8_t *d_text,
     // names phase: as few table slots per warp and step as give every warp of the grid at most one step
     F.scan_w = 8u;
     while (F.scan_w < 32u && (size_t)(t->cap + 1 + F.scan_w - 1) / F.scan_w > (size_t)grid * SF_WARPS) F.scan_w *= 2u;
-    if (ctx->force_scan_w) F.scan_w = (uint32_t)ctx->force_scan_w;
     // KXPU_TRACE_SMALL=1 (debug): SM clocks at the phase boundaries of every CTA, printed per launch
     static const bool trace_on = getenv("KXPU_TRACE_SMALL") != nullptr;
     long long *d_trace = nullptr;
-    if (trace_on && cudaMalloc((void **)&d_trace, (size_t)grid * 128 + (size_t)P.num_chunks * 32) == cudaSuccess) { cudaMemset(d_trace, 0, (size_t)grid * 128 + (size_t)P.num_chunks * 32); P.trace = d_trace; P.F.trace = d_trace + (size_t)grid * 8 + (size_t)P.num_chunks * 4; }
+    if (trace_on && cudaMalloc((void **)&d_trace, (size_t)grid * 64) == cudaSuccess) { cudaMemset(d_trace, 0, (size_t)grid * 64); P.trace = d_trace; }
     {
         KxTimer tm(ctx, KXPU_T_PARSE);
         KX_CUDA(ctx, cudaLaunchCooperativeKernel((const void *)kxsmall::small_load_kernel, dim3(grid), dim3(NT), args, (size_t)WARPS * STG_BYTES, ctx->stream));
         KX_LAUNCHED(ctx);
     }
     if (d_trace) {
-        std::vector<long long> h((size_t)grid * 16 + (size_t)P.num_chunks * 4);
+        std::vector<long long> h((size_t)grid * 8);
         cudaStreamSynchronize(ctx->stream);
         cudaMemcpy(h.data(), d_trace, h.size() * 8, cudaMemcpyDeviceToHost);
         cudaFree(d_trace);
@@ -547,39 +546,6 @@ static int32_t launch_small(kxpu_ctx *ctx, kxpu_table *t, const uint8_t *d_text,
                 mn = std::min(mn, d); mx = std::max(mx, d); sum += d; cnt++;
             }
             if (cnt) fprintf(stderr, " %s %lld/%lld/%lld |", nm[k], mn, sum / cnt, mx);
-        }
-        {   // the slowest CTAs of phase 2 (chunks 8*b .. 8*b+7)
-            std::vector<std::pair<long long, unsigned>> v;
-            for (unsigned b = 0; b < grid; b++) v.push_back({h[b * 8 + 3] - h[b * 8 + 2], b});
-            std::sort(v.rbegin(), v.rend());
-            fprintf(stderr, " slowest phase2 CTAs:");
-            for (int k = 0; k < 6 && k < (int)v.size(); k++) fprintf(stderr, " %u:%lld", v[k].second, v[k].first);
-            // per chunk warp: cycles of phase 2, of its part in front of the folds, fold-list entries, look-back steps
-            std::vector<std::pair<long long, unsigned>> wv;
-            const long long *tw = h.data() + (size_t)grid * 8;
-            for (unsigned c = 0; c < P.num_chunks; c++) wv.push_back({tw[c * 4], c});
-            std::sort(wv.rbegin(), wv.rend());
-            fprintf(stderr, "\n   slowest phase2 warps (chunk: cycles / before folds / entries / look-back steps):");
-            for (int k = 0; k < 10 && k < (int)wv.size(); k++) {
-                const unsigned c = wv[k].second;
-                fprintf(stderr, " %u: %lld/%lld/%lld/%lld |", c, tw[c * 4], tw[c * 4 + 1], tw[c * 4 + 2], tw[c * 4 + 3]);
-            }
-            const unsigned mid = wv[wv.size() / 2].second;
-            fprintf(stderr, " median %u: %lld/%lld/%lld/%lld", mid, tw[mid * 4], tw[mid * 4 + 1], tw[mid * 4 + 2], tw[mid * 4 + 3]);
-            // names phase, thread 0 of every CTA: start(=mark 4 of the kernel) -> scan -> rounds -> claim -> sync -> out -> long lines -> end
-            const long long *tf = h.data() + (size_t)grid * 8 + (size_t)P.num_chunks * 4;
-            static const char *fn[7] = {"scan", "rounds", "sync1+claim", "sync2", "names out+rows", "long lines", "shift+sync3"};
-            fprintf(stderr, "\n   names phase per CTA (thread 0), cycles min/avg/max:");
-            for (int k = 0; k < 7; k++) {
-                long long mn = 1ll << 62, mx = 0, sum = 0, cnt = 0;
-                for (unsigned b = 0; b < grid; b++) {
-                    const long long t1 = tf[b * 8 + k], t0 = k ? tf[b * 8 + k - 1] : h[b * 8 + 4];
-                    if (!t1 || !t0) continue;
-                    const long long d = t1 - t0;
-                    mn = std::min(mn, d); mx = std::max(mx, d); sum += d; cnt++;
-                }
-                if (cnt) fprintf(stderr, " %s %lld/%lld/%lld |", fn[k], mn, sum / cnt, mx);
-            }
         }
         fprintf(stderr, "\n");
     }
@@ -721,7 +687,7 @@ extern "C" int32_t kxpu_pciids_join(kxpu_ctx *ctx, const uint8_t *text, size_t n
     // phase (one TMA bulk copy per 2 KiB chunk, all in flight at once), reads the keys and writes the row handles and
     // the table counters straight to host memory; the call is one launch and one stream synchronisation.
     const uint32_t chunks = (uint32_t)((n + kxparse::CW - 1) / kxparse::CW);
-    if (nq && chunks > 0 && chunks <= small_text_chunks(ctx) && !ctx->no_zero_copy) {
+    if (nq && chunks > 0 && chunks <= small_text_chunks(ctx)) {
         const uint8_t *m_text = (const uint8_t *)kx_mapped_host(text);
         const uint32_t *m_keys = (const uint32_t *)kx_mapped_host(keys);
         int32_t *m_rows = (int32_t *)kx_mapped_host(rows_out);

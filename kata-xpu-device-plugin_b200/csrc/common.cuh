@@ -32,8 +32,6 @@ struct kxpu_ctx {
     bool ev_used[KXPU_T_COUNT] = {};
     int force_rch = 0;         // KXPU_RCH: chunks per parse range (0 = automatic), for tests
     bool no_small = false;     // KXPU_NO_SMALL: never use the cooperative small-text kernel, for tests
-    bool no_zero_copy = false; // KXPU_NO_ZERO_COPY: kxpu_pciids_join always copies its inputs to the device first, for tests
-    int force_scan_w = 0;      // KXPU_SCAN_W: table slots a finalize warp scans per step (8 / 16 / 32; 0 = automatic), for experiments
     int small_chunks = -1;     // chunks the small-text kernel can take (-1: not asked yet)
     bool stage_timing = true;  // per-stage CUDA events (kxpu_last_timings); kxpu_set_stage_timing(ctx, 0) drops them
     uint64_t launches = 0;

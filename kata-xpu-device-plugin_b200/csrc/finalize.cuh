@@ -119,7 +119,6 @@ struct FinalizeParams {
     uint32_t slab_rows_cap;
     uint32_t scan_w;          // table slots a warp scans per step: 8 (latency) or 32 (big tables)
     kxx::SlabTail tail;       // sharded load: header + "slab ready" flags by the last CTA
-    long long *trace;         // debug (KXPU_TRACE_SMALL): [gridDim.x][8] clock64 of thread 0 inside the first step
 };
 
 __device__ __forceinline__ void finalize_store_row(const FinalizeParams &F, uint32_t row, uint32_t slot, uint32_t key, unsigned long long line,
@@ -156,8 +155,6 @@ struct SfEntry {
     uint32_t slot, key;
 };
 constexpr int SF_QCAP = SF_BATCH - 1 + 32;  // what is left of the queue + one scan
-
-#define SF_MARK(k) do { if (F.trace && threadIdx.x == 0 && F.trace[blockIdx.x * 8u + (k)] == 0) F.trace[blockIdx.x * 8u + (k)] = clock64(); } while (0)
 
 __device__ __forceinline__ void select_finalize_body(const FinalizeParams &F, const uint32_t scan_w) {
     __shared__ __align__(16) uint8_t s_raw[SF_WARPS][4][SF_WIN + 16];
@@ -210,7 +207,6 @@ __device__ __forceinline__ void select_finalize_body(const FinalizeParams &F, co
             qn += (uint32_t)__popc(vm);
             __syncwarp();
         }
-        SF_MARK(0);
         const bool have = chunk < nchunks;
         const uint32_t nvalid = qn >= (uint32_t)SF_BATCH ? (uint32_t)SF_BATCH : (have ? 0u : qn);  // rows of this batch: queue[0, nvalid)
         uint32_t my_len = 0;    // lane r (< nvalid): sanitised length of batch row r
@@ -305,15 +301,9 @@ __device__ __forceinline__ void select_finalize_body(const FinalizeParams &F, co
             __syncwarp();  // the next round overwrites the raw windows this round's lanes read from
         }
         __syncwarp();
-        SF_MARK(1);
         // one claim of row handles and of blob space per batch
         uint32_t len_r = (lane < nvalid && !((slow_m >> lane) & 1u)) ? my_len : 0u;
-        uint32_t incl = len_r;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const uint32_t y = __shfl_up_sync(0xffffffffu, incl, d);
-            if (lane >= (uint32_t)d) incl += y;
-        }
+        const uint32_t incl = warp_incl_scan(len_r);
         const uint32_t wtot = __shfl_sync(0xffffffffu, incl, 31);
         if (lane == 0) { s_cnt[wl] = nvalid; s_bytes[wl] = wtot; s_more[wl] = (have || qn > nvalid) ? 1u : 0u; }
         __syncthreads();
@@ -326,9 +316,7 @@ __device__ __forceinline__ void select_finalize_body(const FinalizeParams &F, co
             if (b0 + bytes > F.blob_cap) { F.tab.counters[KX_C_BLOB_OVERFLOW] = 1u; b0 = 0xFFFFFFFFu; }
             s_blob0 = b0;
         }
-        SF_MARK(2);
         __syncthreads();
-        SF_MARK(3);
         uint32_t row0 = s_row0, blob0 = s_blob0, more = 0;
         for (uint32_t k = 0; k < wl; k++) { row0 += s_cnt[k]; if (blob0 != 0xFFFFFFFFu) blob0 += s_bytes[k]; }
 #pragma unroll
@@ -346,7 +334,6 @@ __device__ __forceinline__ void select_finalize_body(const FinalizeParams &F, co
             const SfEntry e = q[lane];
             finalize_store_row(F, row0 + lane, e.slot, e.key, e.line, e.anchor, room ? off_r : 0u, room ? len_r : 0u);
         }
-        SF_MARK(4);
         // long lines (the rest does not end inside the 128-byte window; 19 device lines of pci.ids):
         // the whole warp takes them one at a time -- the line is staged into the (now free) name staging
         // area 32 bytes per step, then sanitised one byte per lane with ballot compaction
@@ -419,7 +406,6 @@ __device__ __forceinline__ void select_finalize_body(const FinalizeParams &F, co
             if (lane == 0) finalize_store_row(F, row0 + r, l_slot, l_key, l_line, l_anchor, ok ? at : 0u, ok ? out_len : 0u);
             __syncwarp();
         }
-        SF_MARK(5);
         // what is left of the queue moves to its front
         {
             const uint32_t rem = qn - nvalid;
@@ -433,7 +419,6 @@ __device__ __forceinline__ void select_finalize_body(const FinalizeParams &F, co
             qn = rem;
         }
         __syncthreads();  // the staging rows and the claim words are reused by the next step
-        SF_MARK(6);
         if (!more) break;
     }
 }

@@ -1,7 +1,8 @@
-// parse_common.cuh -- building blocks of the pci.ids parse kernel (pciids5.cu) and of the
-// kernels behind it (finalize.cuh, comm.cu): chunk geometry, status-word encodings, mbarrier /
-// 1-D TMA bulk copy wrappers, the SWAR newline and hex primitives, shared-window accessors and
-// the table fold ("first occurrence wins", device_plugin.go:237,265).
+// parse_common.cuh -- building blocks of the pci.ids parse kernels (pciids5.cu, small.cuh) and of
+// the kernels behind them (finalize.cuh, comm.cu): chunk geometry, status-word encodings, mbarrier /
+// 1-D TMA bulk copy wrappers and chunk staging, the SWAR newline and hex primitives, line classes,
+// shared-window accessors, the table fold ("first occurrence wins", device_plugin.go:237,265) and
+// the per-warp fold list.
 #pragma once
 #include "common.cuh"
 #include "table.cuh"
@@ -293,12 +294,25 @@ __device__ __forceinline__ uint32_t stage_chunk_manual(const uint8_t *text, unsi
     return n_rel;
 }
 
-// Newline masks and line classes of the chunk staged at shared address st.  Lane owns bytes
-// [32*lane, 32*lane+32) of each KiB half; the two 16-byte pieces are read in a lane-dependent
-// order so that every LDS.128 phase hits all banks.  kh / th: kept / top-level line starts,
-// bit b = the line that starts after a newline at byte b of the lane's window.
-__device__ __forceinline__ void chunk_masks(uint32_t st, uint32_t lane, uint32_t n_rel, uint32_t k7f, uint32_t k0a, uint32_t k80,
-                                            uint32_t (&kh)[2], uint32_t (&th)[2], uint32_t &rawnl) {
+// Stage one chunk (STG_BYTES from src) at shared address st with one bulk copy and wait for it: one
+// copy instead of five dependent 16-byte round trips per lane.  The caller owns the mbarrier `bar`
+// (initialised with count 1) and its phase parity.
+__device__ __forceinline__ void stage_chunk_tma(uint32_t st, const uint8_t *src, uint32_t bar, uint32_t parity, uint32_t lane,
+                                                unsigned long long pol) {
+    if (lane == 0) {
+        mbar_expect_tx_a(bar, STG_BYTES);
+        tma_load_a(st, src, STG_BYTES, bar, pol);
+    }
+    while (!mbar_try_a(bar, parity)) {
+    }
+}
+
+// Newline masks of the chunk staged at shared address st.  Lane owns bytes [32*lane, 32*lane+32)
+// of each KiB half; the two 16-byte pieces are read in a lane-dependent order so that every
+// LDS.128 phase hits all banks.  nl[h] bit b = a line starts after the newline at byte b of the
+// lane's window in KiB half h, trimmed to real line starts (< n_rel).
+__device__ __forceinline__ void nl_masks(uint32_t st, uint32_t lane, uint32_t n_rel, uint32_t k7f, uint32_t k0a, uint32_t k80,
+                                         uint32_t (&nl)[2], uint32_t &rawnl) {
     const uint32_t swz = (lane >> 2) & 1u;
     rawnl = 0;
 #pragma unroll
@@ -307,34 +321,42 @@ __device__ __forceinline__ void chunk_masks(uint32_t st, uint32_t lane, uint32_t
         const uint4 va = lds128(st + o + 16u * swz);
         const uint4 vb = lds128(st + o + 16u * (swz ^ 1u));
         const uint32_t ma = nl_mask16(va, k7f, k0a, k80), mb = nl_mask16(vb, k7f, k0a, k80);
-        uint32_t mm = swz ? (mb | (ma << 16)) : (ma | (mb << 16));
+        const uint32_t m2 = ma | (mb << 16);
+        uint32_t mm = __funnelshift_l(m2, m2, swz << 4);  // swapped read order: swap the halves back
         rawnl |= mm;
-        // a line start at o + 1 + b is real only below n_rel (ragged last chunk)
         if (n_rel <= (uint32_t)CW) mm &= n_rel > o + 1u ? (n_rel - o - 1u >= 32u ? 0xffffffffu : ((1u << (n_rel - o - 1u)) - 1u)) : 0u;
-        // class of the line that starts after each newline, by its first two bytes:
-        //   neither '#' nor '\t': top-level line -- ends the vendor block
-        //     (device_plugin.go:229-236), the only kind locateVendor can match (:265)
-        //   "\t" + non-tab: device line candidate (:237); "\t\t" subsystem, '#' comment: dropped
-        uint32_t km = 0, tm = 0;
-        const uint32_t lp = st + o + 1u;
-        while (mm) {
-            const uint32_t b = (uint32_t)__ffs((int)mm) - 1u;
-            const uint32_t bit = mm & (0u - mm);
-            mm ^= bit;
-            const uint32_t c0 = lds8(lp + b), c1 = lds8(lp + b + 1u);
-            asm("{\n\t.reg .pred p0, pt, pc, pk;\n\t"
-                "setp.eq.u32 p0, %2, 9;\n\t"
-                "setp.ne.and.u32 pt, %2, 35, !p0;\n\t"
-                "setp.ne.and.u32 pc, %3, 9, p0;\n\t"
-                "or.pred pk, pt, pc;\n\t"
-                "@pt or.b32 %0, %0, %4;\n\t"
-                "@pk or.b32 %1, %1, %4;\n\t}"
-                : "+r"(tm), "+r"(km)
-                : "r"(c0), "r"(c1), "r"(bit));
-        }
-        kh[h] = km;
-        th[h] = tm;
+        nl[h] = mm;
     }
+}
+
+// top-level line starts (first byte neither '\t' nor '#': device_plugin.go:229-236) among the line
+// starts m0 / m1 of the lane's two windows (KiB halves), one loop, both loads in flight; lp0 =
+// shared address of the byte after byte 0 of the first window
+__device__ __forceinline__ void tops_of2(uint32_t lp0, uint32_t m0, uint32_t m1, uint32_t &t0, uint32_t &t1) {
+    t0 = t1 = 0;
+    while (m0 | m1) {
+        const uint32_t b0 = m0 & (0u - m0), b1 = m1 & (0u - m1);
+        m0 ^= b0;
+        m1 ^= b1;
+        // an exhausted mask reads the byte in front of the window (31 - clz(0) = -1) and ORs in nothing
+        const uint32_t c0 = lds8(lp0 + (31u - (uint32_t)__clz((int)b0)));
+        const uint32_t c1 = lds8(lp0 + (uint32_t)HALF + (31u - (uint32_t)__clz((int)b1)));
+        if (c0 != 9u && c0 != 35u) t0 |= b0;
+        if (c1 != 9u && c1 != 35u) t1 |= b1;
+    }
+}
+
+// device line candidates ("\t" + non-tab, :237) among the line starts mm of one window; lp =
+// shared address of the byte after the window's byte 0
+__device__ __forceinline__ uint32_t devs_of(uint32_t lp, uint32_t mm) {
+    uint32_t km = 0;
+    while (mm) {
+        const uint32_t bit = mm & (0u - mm);
+        mm ^= bit;
+        const uint32_t a = lp + (31u - (uint32_t)__clz((int)bit));
+        if (lds8(a) == 9u && lds8(a + 1u) != 9u) km |= bit;
+    }
+    return km;
 }
 
 // device lines `m` (bit b: line starts at pbase + b) of the chunk staged at st, all governed by
@@ -348,6 +370,113 @@ __device__ __forceinline__ void fold_lines(const KxTableDev &tab, uint32_t st, u
         const uint32_t p = pbase + b;
         uint32_t dv;
         if (hex4_swar(lds32_unaligned(st + p + 1u), dv)) table_fold(tab, key_hi | dv, cbase + p, anchor, fresh_cnt);
+    }
+}
+
+// inclusive prefix sum of v over the warp (all 32 lanes must call)
+__device__ __forceinline__ uint32_t warp_incl_scan(uint32_t v) {
+    const uint32_t lane = threadIdx.x & 31u;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint32_t y = __shfl_up_sync(0xffffffffu, v, d);
+        if (lane >= (uint32_t)d) v += y;
+    }
+    return v;
+}
+
+constexpr int LIST_CAP = 256;            // entries of a warp's fold list (a 2 KiB chunk of pci.ids has <= 111 device lines)
+constexpr uint32_t LIST_CARRY = 0xfffu;  // governing line = the carry into the chunk
+constexpr uint32_t LIST_DEAD = 0xffeu;   // no alive governing line
+
+// Fold the device lines of the chunk staged at st (global offset cbase) that have an alive governing
+// line (all 32 lanes must call).  Per lane and KiB half h: kh[h] the line starts that matter (device
+// line candidates and top-level lines), th[h] the top-level lines among them, at[h] the alive ones
+// among those, gov[h] the governing line in front of the window: the position of an alive top-level
+// line of the chunk, LIST_CARRY (the carry: vendor carry_hi >> 16, anchor carry_anchor) or LIST_DEAD.
+// Every device line to fold becomes one entry (line position | governing position << 12) of the
+// warp's list (LIST_CAP words of shared memory; a chunk with more lines takes several passes), and
+// the list is folded two entries per lane and round with their probe steps in flight together
+// (`claim`: table_fold_claim2, for an L2-resident table) or one per lane with the load-first
+// table_fold (a table in DRAM).  Folding straight from the windows left a lane's table inserts --
+// two dependent L2 round trips each -- serialised: ~10 in a row for a chunk of short lines.
+__device__ __forceinline__ void fold_list(const KxTableDev &tab, uint32_t *list, uint32_t st, unsigned long long cbase,
+                                          const uint32_t (&kh)[2], const uint32_t (&th)[2], const uint32_t (&at)[2],
+                                          const uint32_t (&gov)[2], uint32_t carry_hi, unsigned long long carry_anchor, bool claim,
+                                          uint32_t &fresh_cnt) {
+    const uint32_t lane = threadIdx.x & 31u;
+    uint32_t mine = 0;
+    for (int h = 0; h < 2; h++) {
+        // lines in front of the window's first top-level line count iff gov is alive, those behind an alive top always
+        const uint32_t dl = kh[h] & ~th[h];
+        const uint32_t first = th[h] & (0u - th[h]);
+        const uint32_t pre = dl & (first ? first - 1u : 0xffffffffu);
+        if (gov[h] != LIST_DEAD) mine += (uint32_t)__popc(pre);
+        uint32_t t = th[h];
+        while (t) {
+            const uint32_t bit = t & (0u - t);
+            t ^= bit;
+            const uint32_t nxt = t & (0u - t);
+            if (at[h] & bit) mine += (uint32_t)__popc(dl & ~(bit | (bit - 1u)) & (nxt ? nxt - 1u : 0xffffffffu));
+        }
+    }
+    const uint32_t incl = warp_incl_scan(mine);
+    const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+    const uint32_t off = incl - mine;
+    auto entry = [&](uint32_t e, uint32_t &key, unsigned long long &line, unsigned long long &anchor) -> bool {
+        const uint32_t p = e & 0xfffu, gp = e >> 12;
+        uint32_t key_hi = carry_hi, dv;
+        anchor = carry_anchor;
+        if (gp != LIST_CARRY) {
+            uint32_t val;
+            hex4_swar(lds32_unaligned(st + gp), val);  // an alive line: its id parsed fine before
+            key_hi = val << 16;
+            anchor = cbase + gp;
+        }
+        line = cbase + p;
+        const bool ok = hex4_swar(lds32_unaligned(st + p + 1u), dv);
+        key = key_hi | dv;
+        return ok;
+    };
+    for (uint32_t base = 0; base < total; base += (uint32_t)LIST_CAP) {  // one pass unless the chunk has > LIST_CAP lines
+        // my entries whose list index falls into [base, base + LIST_CAP)
+        {
+            uint32_t idx = off;
+            for (int h = 0; h < 2; h++) {
+                const uint32_t pbase = (uint32_t)h * HALF + lane * 32u + 1u;
+                uint32_t g = gov[h];
+                uint32_t m = kh[h];
+                while (m) {
+                    const uint32_t bit = m & (0u - m);
+                    m ^= bit;
+                    const uint32_t p = pbase + (31u - (uint32_t)__clz((int)bit));
+                    if (th[h] & bit) {
+                        g = (at[h] & bit) ? p : LIST_DEAD;
+                    } else if (g != LIST_DEAD) {
+                        if (idx >= base && idx < base + (uint32_t)LIST_CAP) list[idx - base] = p | (g << 12);
+                        idx++;
+                    }
+                }
+            }
+        }
+        __syncwarp();
+        const uint32_t cnt = total - base < (uint32_t)LIST_CAP ? total - base : (uint32_t)LIST_CAP;
+        if (claim) {
+            for (uint32_t i = lane; i < cnt; i += 64u) {
+                uint32_t k0, k1 = 0;
+                unsigned long long l0, a0, l1 = 0, a1 = 0;
+                bool v0 = entry(list[i], k0, l0, a0);
+                bool v1 = i + 32u < cnt && entry(list[i + 32u], k1, l1, a1);
+                if (!v0 && v1) { k0 = k1; l0 = l1; a0 = a1; v0 = true; v1 = false; }
+                if (v0) table_fold_claim2(tab, k0, l0, a0, v1, k1, l1, a1, fresh_cnt);
+            }
+        } else {
+            for (uint32_t i = lane; i < cnt; i += 32u) {
+                uint32_t k;
+                unsigned long long l, a;
+                if (entry(list[i], k, l, a)) table_fold(tab, k, l, a, fresh_cnt);
+            }
+        }
+        __syncwarp();
     }
 }
 

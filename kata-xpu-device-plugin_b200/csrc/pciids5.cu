@@ -61,68 +61,6 @@ struct Params5 {
     kxx::XaParams xa;
 };
 
-
-// Newline masks of the chunk staged at shared address st (see kxparse::chunk_masks for the
-// window layout): nl[h] bit b = a line starts after the newline at byte b of the lane's window in
-// KiB half h, trimmed to real line starts (< n_rel).
-__device__ __forceinline__ void nl_masks(uint32_t st, uint32_t lane, uint32_t n_rel, uint32_t k7f, uint32_t k0a, uint32_t k80,
-                                         uint32_t (&nl)[2], uint32_t &rawnl) {
-    const uint32_t swz = (lane >> 2) & 1u;
-    rawnl = 0;
-#pragma unroll
-    for (int h = 0; h < 2; h++) {
-        const uint32_t o = (uint32_t)h * HALF + lane * 32u;
-        const uint4 va = lds128(st + o + 16u * swz);
-        const uint4 vb = lds128(st + o + 16u * (swz ^ 1u));
-        const uint32_t ma = nl_mask16(va, k7f, k0a, k80), mb = nl_mask16(vb, k7f, k0a, k80);
-        const uint32_t m2 = ma | (mb << 16);
-        uint32_t mm = __funnelshift_l(m2, m2, swz << 4);  // swapped read order: swap the halves back
-        rawnl |= mm;
-        if (n_rel <= (uint32_t)CW) mm &= n_rel > o + 1u ? (n_rel - o - 1u >= 32u ? 0xffffffffu : ((1u << (n_rel - o - 1u)) - 1u)) : 0u;
-        nl[h] = mm;
-    }
-}
-
-// top-level line starts among the line starts mm of one window (first byte neither '\t' nor
-// '#': device_plugin.go:229-236); lp = shared address of the byte after the window's byte 0
-__device__ __forceinline__ uint32_t tops_of(uint32_t lp, uint32_t mm) {
-    uint32_t tm = 0;
-    while (mm) {
-        const uint32_t bit = mm & (0u - mm);
-        mm ^= bit;
-        const uint32_t c0 = lds8(lp + (31u - (uint32_t)__clz((int)bit)));
-        if (c0 != 9u && c0 != 35u) tm |= bit;
-    }
-    return tm;
-}
-
-// the same for the lane's two windows (KiB halves) at once: one loop, both loads in flight
-__device__ __forceinline__ void tops_of2(uint32_t lp0, uint32_t m0, uint32_t m1, uint32_t &t0, uint32_t &t1) {
-    t0 = t1 = 0;
-    while (m0 | m1) {
-        const uint32_t b0 = m0 & (0u - m0), b1 = m1 & (0u - m1);
-        m0 ^= b0;
-        m1 ^= b1;
-        // an exhausted mask reads the byte in front of the window (31 - clz(0) = -1) and ORs in nothing
-        const uint32_t c0 = lds8(lp0 + (31u - (uint32_t)__clz((int)b0)));
-        const uint32_t c1 = lds8(lp0 + (uint32_t)HALF + (31u - (uint32_t)__clz((int)b1)));
-        if (c0 != 9u && c0 != 35u) t0 |= b0;
-        if (c1 != 9u && c1 != 35u) t1 |= b1;
-    }
-}
-
-// device line candidates ("\t" + non-tab, :237) among the line starts mm of one window
-__device__ __forceinline__ uint32_t devs_of(uint32_t lp, uint32_t mm) {
-    uint32_t km = 0;
-    while (mm) {
-        const uint32_t bit = mm & (0u - mm);
-        mm ^= bit;
-        const uint32_t a = lp + (31u - (uint32_t)__clz((int)bit));
-        if (lds8(a) == 9u && lds8(a + 1u) != 9u) km |= bit;
-    }
-    return km;
-}
-
 __global__ void __launch_bounds__(NT, 4) parse_kernel_v5(const Params5 P) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     WarpSmem5 *W = reinterpret_cast<WarpSmem5 *>(smem_raw);
@@ -420,12 +358,7 @@ __global__ void __launch_bounds__(256) resolve_ranges_kernel(const Params5 P) {
                        P.tab.vendor_first[(uint32_t)(carry >> 44) & 0xffffu] >= (carry & CV_ANCHOR_MASK);  // vendor_first is final here
     // queue space: one atomic per warp (in a text without repeated blocks every range queues its chunks)
     const uint32_t mine = alive ? nlead : 0u;
-    uint32_t incl = mine;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, incl, d);
-        if (lane >= (uint32_t)d) incl += y;
-    }
+    const uint32_t incl = warp_incl_scan(mine);
     const uint32_t tot = __shfl_sync(0xffffffffu, incl, 31);
     uint32_t at0 = 0;
     if (lane == 0 && tot) at0 = atomicAdd(&P.tab.counters[KX_C_DEFER], tot);
@@ -437,11 +370,12 @@ __global__ void __launch_bounds__(256) resolve_ranges_kernel(const Params5 P) {
 }
 
 // Resolve, step 2: one warp per queued chunk stages it again and folds its head lines (the
-// device lines in front of its first top-level line) under the range's governing line.
-__global__ void __launch_bounds__(RES_WARPS * 32) resolve_chunks_kernel(const Params5 P) {
+// device lines in front of its first top-level line) under the range's governing line.  Six CTAs
+// per SM (40 registers): left to itself ptxas trades spills in the task loop for occupancy.
+__global__ void __launch_bounds__(RES_WARPS * 32, 6) resolve_chunks_kernel(const Params5 P) {
     __shared__ __align__(16) uint8_t stg[RES_WARPS][STG_BYTES];
     __shared__ __align__(8) unsigned long long bars[RES_WARPS];
-    __shared__ uint16_t plist[RES_WARPS][704];  // a 2 KiB chunk holds at most 683 candidate lines ("\tX\n")
+    __shared__ uint32_t s_list[RES_WARPS][LIST_CAP];
     if (blockIdx.x >= P.task_ctas) {
         // phase A of the sharded load: these CTAs push slices of the shard's vendor minima into every rank's region while
         // the others fold; the one that finishes last adds cut-off and status and raises the flags (the barrier +
@@ -473,6 +407,8 @@ __global__ void __launch_bounds__(RES_WARPS * 32) resolve_chunks_kernel(const Pa
     const unsigned long long pol = l2_evict_first_policy();
     const uint32_t n_tasks = P.tab.counters[KX_C_DEFER];
     uint32_t par = 0, nfresh = 0;
+    // L2-resident table: claim first (one round trip per probe step); a table in DRAM: load first -- measured 2.5x
+    // faster there (12.4 M keys, 1 GB table: 0.55 ms against 1.4 ms)
     const bool small_tab = P.tab.cap <= (1u << 20);
     uint32_t it = 0;
     for (uint32_t t = blockIdx.x * RES_WARPS + w; t < n_tasks; t += P.task_ctas * RES_WARPS, it++) {
@@ -481,66 +417,25 @@ __global__ void __launch_bounds__(RES_WARPS * 32) resolve_chunks_kernel(const Pa
         const uint32_t gg = P.tasks[t];
         uint32_t n_rel = CW + 1;
         if (gg < P.tma_limit) {
-            // one bulk copy instead of five dependent 16-byte round trips per lane
-            if (lane == 0) {
-                mbar_expect_tx_a(bar, STG_BYTES);
-                tma_load_a(st, P.text + (unsigned long long)gg * CW, STG_BYTES, bar, pol);
-            }
-            while (!mbar_try_a(bar, par)) {
-            }
+            stage_chunk_tma(st, P.text + (unsigned long long)gg * CW, bar, par, lane, pol);
             par ^= 1u;
         } else {
             n_rel = stage_chunk_manual(P.text, P.n, gg, lane, stg[w]);
         }
         const unsigned long long cc = P.range_carry[gg / P.rch];
-        const uint32_t key_hi = ((uint32_t)(cc >> 44) & 0xffffu) << 16;
-        const unsigned long long anchor = cc & CV_ANCHOR_MASK;
-        uint32_t kh[2], th[2], rawnl;
-        chunk_masks(st, lane, n_rel, k7f, k0a, k80, kh, th, rawnl);
+        uint32_t nl[2], th[2], rawnl;
+        nl_masks(st, lane, n_rel, k7f, k0a, k80, nl, rawnl);
+        tops_of2(st + lane * 32u + 1u, nl[0], nl[1], th[0], th[1]);
         const uint32_t bal0 = __ballot_sync(0xffffffffu, th[0] != 0u);
         const uint32_t bal1 = __ballot_sync(0xffffffffu, th[1] != 0u);
-        const uint32_t pre0 = kh[0] & ~th[0] & (th[0] ? (th[0] & (0u - th[0])) - 1u : 0xffffffffu);
-        const uint32_t pre1 = kh[1] & ~th[1] & (th[1] ? (th[1] & (0u - th[1])) - 1u : 0xffffffffu);
-        const unsigned long long cbase = P.base + (unsigned long long)gg * CW;
-        // The head lines become a list of line positions, folded one per lane and round: straight from the
-        // windows a lane with several short lines ran its table inserts (two dependent round trips each) in a row.
-        const uint32_t m0 = (bal0 & lt_mask) == 0u ? pre0 : 0u;
-        const uint32_t m1 = (bal0 == 0u && (bal1 & lt_mask) == 0u) ? pre1 : 0u;
-        const uint32_t mine = (uint32_t)__popc(m0) + (uint32_t)__popc(m1);
-        uint32_t incl = mine;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const uint32_t y = __shfl_up_sync(0xffffffffu, incl, d);
-            if (lane >= (uint32_t)d) incl += y;
-        }
-        const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
-        {
-            uint32_t idx = incl - mine;
-            for (uint32_t m = m0; m; m &= m - 1u) plist[w][idx++] = (uint16_t)(lane * 32u + 1u + (uint32_t)__ffs((int)m) - 1u);
-            for (uint32_t m = m1; m; m &= m - 1u) plist[w][idx++] = (uint16_t)((uint32_t)HALF + lane * 32u + 1u + (uint32_t)__ffs((int)m) - 1u);
-        }
-        __syncwarp();
-        if (small_tab) {
-            // L2-resident table: claim first (one round trip per probe step), two lines per lane and round with their
-            // probe steps in flight together
-            for (uint32_t i = lane; i < total; i += 64u) {
-                uint32_t d0, d1 = 0;
-                const uint32_t p0 = plist[w][i], p1 = i + 32u < total ? plist[w][i + 32u] : 0u;
-                bool v0 = hex4_swar(lds32_unaligned(st + p0 + 1u), d0);
-                bool v1 = i + 32u < total && hex4_swar(lds32_unaligned(st + p1 + 1u), d1);
-                uint32_t q0 = p0, q1 = p1;
-                if (!v0 && v1) { d0 = d1; q0 = p1; v0 = true; v1 = false; }
-                if (v0) table_fold_claim2(P.tab, key_hi | d0, cbase + q0, anchor, v1, key_hi | d1, cbase + q1, anchor, nfresh);
-            }
-        } else {
-            // a table in DRAM: load first -- measured 2.5x faster there (12.4 M keys, 1 GB table: 0.55 ms against 1.4 ms)
-            for (uint32_t i = lane; i < total; i += 32u) {
-                const uint32_t p = plist[w][i];
-                uint32_t dv;
-                if (hex4_swar(lds32_unaligned(st + p + 1u), dv)) table_fold(P.tab, key_hi | dv, cbase + p, anchor, nfresh);
-            }
-        }
-        __syncwarp();
+        // head lines: the device lines of the windows in front of the chunk's first top-level line
+        const uint32_t pre0 = nl[0] & (th[0] ? (th[0] & (0u - th[0])) - 1u : 0xffffffffu);
+        const uint32_t pre1 = nl[1] & (th[1] ? (th[1] & (0u - th[1])) - 1u : 0xffffffffu);
+        const uint32_t head[2] = {(bal0 & lt_mask) == 0u ? devs_of(st + lane * 32u + 1u, pre0) : 0u,
+                                  (bal0 == 0u && (bal1 & lt_mask) == 0u) ? devs_of(st + (uint32_t)HALF + lane * 32u + 1u, pre1) : 0u};
+        const uint32_t none[2] = {0u, 0u}, gov[2] = {LIST_CARRY, LIST_CARRY};
+        fold_list(P.tab, s_list[w], st, P.base + (unsigned long long)gg * CW, head, none, none, gov, ((uint32_t)(cc >> 44) & 0xffffu) << 16,
+                  cc & CV_ANCHOR_MASK, small_tab, nfresh);
         flush_fresh(P.tab, nfresh);
     }
 }

@@ -17,9 +17,6 @@
 namespace kxsmall {
 
 using namespace kxparse;
-using kxparse5::devs_of;
-using kxparse5::nl_masks;
-using kxparse5::tops_of2;
 
 struct SmallParams {
     const uint8_t *text;
@@ -48,10 +45,6 @@ __device__ __forceinline__ void grid_barrier(uint32_t *ctr, uint32_t target) {
     __syncthreads();
 }
 
-constexpr int LIST_CAP = 256;              // entries of a warp's fold list (a 2 KiB chunk of pci.ids has <= 111 device lines)
-constexpr uint32_t LIST_CARRY = 0xfffu;    // governing line = the carry into the chunk
-constexpr uint32_t LIST_DEAD = 0xffeu;     // no alive governing line
-
 #define KX_SMALL_MARK(k) do { if (P.trace && threadIdx.x == 0) P.trace[blockIdx.x * 8u + (k)] = clock64(); } while (0)
 
 __global__ void __launch_bounds__(NT, 4) small_load_kernel(const SmallParams P) {
@@ -75,16 +68,12 @@ __global__ void __launch_bounds__(NT, 4) small_load_kernel(const SmallParams P) 
     if (have) {
         const uint8_t *src = P.text_src ? P.text_src : P.text;
         if (g < P.tma_limit) {
-            const uint32_t bar = smem_u32(&bars[w]);
             if (lane == 0) {
                 mbar_init(&bars[w], 1);
                 asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-                mbar_expect_tx_a(bar, STG_BYTES);
-                tma_load_a(st, src + cbase, STG_BYTES, bar, l2_evict_first_policy());
             }
             __syncwarp();
-            while (!mbar_try_a(bar, 0)) {
-            }
+            stage_chunk_tma(st, src + cbase, smem_u32(&bars[w]), 0u, lane, l2_evict_first_policy());
         } else {
             n_rel = stage_chunk_manual(src, P.n, g, lane, stage);
         }
@@ -153,15 +142,11 @@ __global__ void __launch_bounds__(NT, 4) small_load_kernel(const SmallParams P) 
     // ---------------------------------------------------------------- phase 2
     uint32_t nfresh = 0;
     if (have) {
-        const long long w_t0 = P.trace ? clock64() : 0;
-        long long w_t1 = 0;
-        uint32_t lb_iters = 0;
         // governing line at the start of the chunk: nearest published prefix in front of it
         unsigned long long carry = 0;
         if (g > 0u) {
             long long q0 = (long long)g - 1;
             for (;;) {
-                lb_iters++;
                 const long long q = q0 - lane;
                 const unsigned long long sv = q >= 0 ? P.state[q] : ST_NONE;
                 const uint32_t m = __ballot_sync(0xffffffffu, (sv & ST_MASK) == ST_PREFIX);
@@ -203,91 +188,10 @@ __global__ void __launch_bounds__(NT, 4) small_load_kernel(const SmallParams P) 
         const uint32_t cv = (uint32_t)(carry >> 44) & 0xffffu;
         const unsigned long long canchor = carry & CV_ANCHOR_MASK;
         const bool carry_alive = (carry & CV_HAS_TOP) && (carry & CV_VOK) && tab.vendor_first[cv] == canchor;
-        // Every device line under an alive governing line becomes one entry (line position | position of the
-        // governing line << 12, LIST_CARRY = the carry) of the warp's list; the list is then folded one entry
-        // per lane and round.  Folding straight from the windows left the table inserts -- two dependent L2
-        // round trips each -- serialised per lane: ~10 in a row for a chunk of short lines (18 us of 53).
-        auto gov_in = [&](int h) -> uint32_t {  // governing line in front of window h
-            return cin[h] == P_NONE ? (carry_alive ? LIST_CARRY : LIST_DEAD) : ((cin[h] >> 31) ? (cin[h] & 0x7fffu) : LIST_DEAD);
-        };
-        uint32_t mine = 0;
-        for (int h = 0; h < 2; h++) {
-            // lines in front of the window's first top-level line count iff gov_in is alive, those behind an alive top always
-            const uint32_t dl = kh[h] & ~th[h];
-            const uint32_t first = th[h] & (0u - th[h]);
-            const uint32_t pre = dl & (first ? first - 1u : 0xffffffffu);
-            if (gov_in(h) != LIST_DEAD) mine += (uint32_t)__popc(pre);
-            uint32_t t = th[h];
-            while (t) {
-                const uint32_t bit = t & (0u - t);
-                t ^= bit;
-                const uint32_t nxt = t & (0u - t);
-                if (at[h] & bit) mine += (uint32_t)__popc(dl & ~(bit | (bit - 1u)) & (nxt ? nxt - 1u : 0xffffffffu));
-            }
-        }
-        uint32_t incl = mine;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const uint32_t y = __shfl_up_sync(0xffffffffu, incl, d);
-            if (lane >= (uint32_t)d) incl += y;
-        }
-        const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
-        const uint32_t off = incl - mine;
-        uint32_t *list = s_list[w];
-        if (P.trace) w_t1 = clock64();
-        for (uint32_t base = 0; base < total; base += (uint32_t)LIST_CAP) {  // one pass unless the chunk has > LIST_CAP lines
-            // my entries whose list index falls into [base, base + LIST_CAP)
-            {
-                uint32_t idx = off;
-                for (int h = 0; h < 2; h++) {
-                    const uint32_t pbase = (uint32_t)h * HALF + lane * 32u + 1u;
-                    uint32_t gov = gov_in(h);
-                    uint32_t m = kh[h];
-                    while (m) {
-                        const uint32_t bit = m & (0u - m);
-                        m ^= bit;
-                        const uint32_t p = pbase + (31u - (uint32_t)__clz((int)bit));
-                        if (th[h] & bit) {
-                            gov = (at[h] & bit) ? p : LIST_DEAD;
-                        } else if (gov != LIST_DEAD) {
-                            if (idx >= base && idx < base + (uint32_t)LIST_CAP) list[idx - base] = p | (gov << 12);
-                            idx++;
-                        }
-                    }
-                }
-            }
-            __syncwarp();
-            const uint32_t cnt = total - base < (uint32_t)LIST_CAP ? total - base : (uint32_t)LIST_CAP;
-            // two entries per lane and round, their probe steps in flight together
-            auto entry = [&](uint32_t e, uint32_t &key, unsigned long long &line, unsigned long long &anchor) -> bool {
-                const uint32_t p = e & 0xfffu, gp = e >> 12;
-                uint32_t key_hi = cv << 16, dv;
-                anchor = canchor;
-                if (gp != LIST_CARRY) {
-                    uint32_t val;
-                    hex4_swar(lds32_unaligned(st + gp), val);  // an alive line: its id parsed fine before
-                    key_hi = val << 16;
-                    anchor = cbase + gp;
-                }
-                line = cbase + p;
-                const bool ok = hex4_swar(lds32_unaligned(st + p + 1u), dv);
-                key = key_hi | dv;
-                return ok;
-            };
-            for (uint32_t i = lane; i < cnt; i += 64u) {
-                uint32_t k0, k1 = 0;
-                unsigned long long l0, a0, l1 = 0, a1 = 0;
-                bool v0 = entry(list[i], k0, l0, a0);
-                bool v1 = i + 32u < cnt && entry(list[i + 32u], k1, l1, a1);
-                if (!v0 && v1) { k0 = k1; l0 = l1; a0 = a1; v0 = true; v1 = false; }
-                if (v0) table_fold_claim2(tab, k0, l0, a0, v1, k1, l1, a1, nfresh);
-            }
-            __syncwarp();
-        }
-        if (P.trace && lane == 0) {
-            long long *tw = P.trace + (size_t)gridDim.x * 8u + (size_t)g * 4u;
-            tw[0] = clock64() - w_t0; tw[1] = w_t1 - w_t0; tw[2] = total; tw[3] = lb_iters;
-        }
+        uint32_t gov[2];  // governing line in front of window h
+        for (int h = 0; h < 2; h++)
+            gov[h] = cin[h] == P_NONE ? (carry_alive ? LIST_CARRY : LIST_DEAD) : ((cin[h] >> 31) ? (cin[h] & 0x7fffu) : LIST_DEAD);
+        fold_list(tab, s_list[w], st, cbase, kh, th, at, gov, cv << 16, canchor, true, nfresh);
     }
     flush_fresh(tab, nfresh);
     KX_SMALL_MARK(3);

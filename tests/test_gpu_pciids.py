@@ -461,5 +461,8 @@ def test_small_texts_through_the_big_text_kernels(oracle, pci_text, monkeypatch)
             check_text(k, oracle, pci_text[:n])
         rng = np.random.default_rng(8)
         check_text(k, oracle, _big_random_text(rng, 6000, 80, 0.4), extra_keys=[0x00010001, 0x00630000])
+        # every chunk of the device lines is a range head with ~340 lines: resolve_chunks_kernel folds its list in passes
+        text = b"10de  NV\n" + b"\n".join(b"\t%04x" % d for d in range(3000)) + b"\n\n\n\n" * 3000 + b"\t0001  late\n"
+        check_text(k, oracle, text, extra_keys=[0x10de0000, 0x10de0bb7, 0x10de0001])
     finally:
         k.close()
